@@ -2,7 +2,12 @@
 """bench.py -- denoising steps/sec of the U-Net hot path (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|torch-gpu] [--workload cfg3|cfg2a|cfg1|cfg5]
+                    [--dump-outputs DIR]
     (N > 1: launched by torch.distributed.run, one rank per GPU)
+
+--dump-outputs DIR writes what the last timed step returned as DIR/image.npy in float32: the sampling image x_{t-1} (with
+N > 1, the ranks' shards as the timed path gathers them: finalized to [0, 1], one global batch).  Inputs, weights and the
+in-graph noise are seeded, so two builds run with the same arguments can be compared output for output.
 
 Headline workload (default = BASELINE.json configs[2], the configuration the metric's target is quoted on; fits one GPU):
     cfg3: SR U-Net 64->256, `Unet(**Super.defaults, lowres_cond=True, text_embed_dim=768)`, 256x256, batch 32 per GPU
@@ -328,7 +333,11 @@ def main():
     ap.add_argument("--profiler-range", action="store_true",
                     help="cudaProfilerStart/Stop around the timed steps (for `ncu --profile-from-start off`: launch lists of exactly K steps)")
     ap.add_argument("--gn-f16", action="store_true", help="GroupNorm inputs in fp16 (faster, 1.05e-3 instead of 9e-4 rel-L2)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the output of the last timed step to DIR/image.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -505,6 +514,8 @@ def main():
         assert torch.isfinite(state()).all(), "non-finite output"
         peak_mem = torch.cuda.max_memory_allocated(dev) / 2 ** 30
         print(f"[bench] device-resident: {ms / args.steps:.2f} ms/step", file=sys.stderr, flush=True)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"image": gathered if world > 1 else state()})
 
         if args.kernel_table and rank == 0:
             kernel_table(lambda: [replay() for _ in range(3)], 3, args.kernel_table)
@@ -833,6 +844,22 @@ def main():
     print(json.dumps(result))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Each array as <path>/<name>.npy in float32.  An array beyond DUMP_BYTES is written as a fixed seeded sample of
+    its elements (flat, in index order), the same sample on every run."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() * 4 > DUMP_BYTES:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_BYTES // 4].sort().values
+            t = t.flatten()[idx.to(t.device)]
+        np.save(os.path.join(path, f"{name}.npy"), t.cpu().numpy())
 
 
 def kernel_table(fn, steps, path):

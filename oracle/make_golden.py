@@ -1,7 +1,11 @@
-"""TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.pt by running the UNMODIFIED reference (oracle/reference.py)
-on the CPU in this container.  Re-run with:  python oracle/make_golden.py
-The fixtures pin (a) oracle/restatement.py and (b) the CUDA path on the GPU box, where /root/reference is absent.
+"""TEST INFRASTRUCTURE ONLY -- generates tests/golden/* by running the UNMODIFIED reference (oracle/reference.py)
+on the CPU.  Re-run with:  python oracle/make_golden.py [train | reference]
+The fixtures pin (a) oracle/restatement.py and (b) the CUDA path, on machines where the reference is absent.
+`signature_table` and `state_dict_digest` are shared with the tests that read the `reference` fixtures.
 """
+import hashlib
+import inspect
+import json
 import os
 import sys
 
@@ -12,6 +16,9 @@ sys.path.insert(0, ROOT)
 from oracle import reference  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
+# torch's fp32 CPU kernels split their sums by the intra-op thread count, so the last bits of every fixture depend on it
+# (and on the ISA: AVX-512).  The fixtures were made with this many threads; the bit-exact tests run with it too.
+CPU_THREADS = 8
 
 
 def _inputs(b, s, L, E, seed, lowres):
@@ -208,12 +215,95 @@ def train_case():
                     cond_drop_prob=0.15), os.path.join(OUT, "train_tiny.pt"))
 
 
+def signature_table(unet_mod, imagen_mod, diffusion_mod):
+    """Parameter lists (name, kind, repr of the default) of the public constructors / entry points and the U-Net
+    presets' defaults (repr), as JSON-ready lists and strings."""
+    def params(f):
+        return [[p.name, p.kind.name, "<empty>" if p.default is inspect.Parameter.empty else repr(p.default)]
+                for p in inspect.signature(f).parameters.values()]
+    return {"Unet.__init__": params(unet_mod.Unet.__init__), "Imagen.__init__": params(imagen_mod.Imagen.__init__),
+            "GaussianDiffusion.__init__": params(diffusion_mod.GaussianDiffusion.__init__),
+            "Unet.forward": params(unet_mod.Unet.forward), "Imagen.sample": params(imagen_mod.Imagen.sample),
+            "presets": {c: repr(getattr(unet_mod, c).defaults) for c in ("Base", "Super", "BaseTest", "SuperTest")}}
+
+
+def state_dict_digest(sd):
+    """SHA-256 over a state dict's names, dtypes, shapes and bytes (in order): pins weights too large to store."""
+    h = hashlib.sha256()
+    for k, v in sd.items():
+        h.update(f"{k}:{v.dtype}:{tuple(v.shape)};".encode())
+        h.update(v.detach().cpu().contiguous().numpy().tobytes())
+    return h.hexdigest()
+
+
+# inputs of the fixtures below; the tests rebuild them from the same seeds
+LIVE_UNET_CFGS = [
+    (dict(dim=32, dim_mults=(1, 2), attend_at_middle=True, text_embed_dim=768), 32, False),
+    (dict(dim=32, dim_mults=(1, 2), lowres_cond=True, memory_efficient=True, num_resnet_blocks=(1, 2),
+          layer_attns=(False, True), layer_cross_attns=(False, True)), 32, True),
+]
+RESIZE_CASES = [(64, 256, "reflect", None), (16, 64, "reflect", (0., 1.)), (128, 64, "reflect", (-1., 1.)),
+                (24, 36, "constant", None), (32, 128, "edge", None)]
+RESIZE_SAMPLE = 4096
+
+
+def live_unet_inputs(cfg, s, lowres):
+    g = torch.Generator().manual_seed(7)
+    x = torch.randn(2, 3, s, s, generator=g)
+    te = torch.randn(2, 20, cfg.get("text_embed_dim", 512), generator=g)
+    tm = torch.ones(2, 20, dtype=torch.bool)
+    tm[1, 5:] = False
+    kw = dict(text_embeds=te, text_mask=tm)
+    if lowres:
+        kw.update(lowres_cond_img=torch.randn(2, 3, s, s, generator=g), lowres_noise_times=torch.tensor([200, 3]))
+    return x, torch.tensor([999, 0]), kw
+
+
+def resize_input(n_in):
+    return torch.rand(2, 3, n_in, n_in, generator=torch.Generator().manual_seed(n_in)) * 2 - 0.5
+
+
+def reference_cases():
+    """What the tests used to compare against the live reference: its signatures (signatures.json), its U-Net forward
+    at two dim-32 configs (unet_dim32.pt: outputs + digest of the seed-0 weights, 6-9 MB each, which the test rebuilds)
+    and its inter-stage resize helper (resize.pt: a fixed seeded sample of each output plus the full-output sum)."""
+    import minimagen.Unet as RU
+    import minimagen.Imagen as RI
+    import minimagen.diffusion_model as RD
+    ref = sys.modules["minimagen"]
+    with open(os.path.join(OUT, "signatures.json"), "w") as f:
+        json.dump(signature_table(RU, RI, RD), f, indent=1)
+        f.write("\n")
+    cases = []
+    for cfg, s, lowres in LIVE_UNET_CFGS:
+        torch.manual_seed(0)
+        r = RU.Unet(**cfg).eval()
+        x, t, kw = live_unet_inputs(cfg, s, lowres)
+        with torch.no_grad():
+            outs = {cdp: r(x, t, cond_drop_prob=cdp, **kw) for cdp in (0., 1.)}
+        cases.append(dict(cfg=cfg, weights_sha256=state_dict_digest(r.state_dict()), outs=outs))
+    torch.save(cases, os.path.join(OUT, "unet_dim32.pt"))
+    res = {}
+    for n_in, n_out, pad, clamp in RESIZE_CASES:
+        want = ref.helpers.resize_image_to(resize_input(n_in), n_out, clamp_range=clamp, pad_mode=pad)
+        n = want.numel()
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:min(n, RESIZE_SAMPLE)].sort().values
+        res[(n_in, n_out, pad, clamp)] = dict(shape=tuple(want.shape), idx=idx.int(), values=want.flatten()[idx].clone(),
+                                              sum=want.double().sum().item())
+    torch.save(res, os.path.join(OUT, "resize.pt"))
+    print("reference cases: unet_dim32", [c["weights_sha256"][:12] for c in cases], "resize", len(res))
+
+
 if __name__ == "__main__":
     reference.load()
+    torch.set_num_threads(CPU_THREADS)
     os.makedirs(OUT, exist_ok=True)
     from minimagen.Unet import BaseTest, SuperTest
     if len(sys.argv) > 1 and sys.argv[1] == "train":
         train_case()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "reference":
+        reference_cases()
         sys.exit(0)
     unet_case("unet_tiny_base", dict(BaseTest.defaults), 64, False)
     unet_case("unet_tiny_sr", dict(SuperTest.defaults, lowres_cond=True), 64, True)
@@ -221,3 +311,4 @@ if __name__ == "__main__":
     sample_case()
     cascade_case()
     train_case()
+    reference_cases()

@@ -30,6 +30,17 @@ def load_golden(name):
 
 
 @pytest.fixture
+def golden_threads():
+    """Bit-exact CPU comparisons with the goldens run with the intra-op thread count the goldens were made with: torch's
+    fp32 CPU kernels split their sums by it, so the last bits depend on it.  Restored afterwards."""
+    from oracle.make_golden import CPU_THREADS
+    prev = torch.get_num_threads()
+    torch.set_num_threads(CPU_THREADS)
+    yield
+    torch.set_num_threads(prev)
+
+
+@pytest.fixture
 def emu():
     """Install the torch emulation of the ops interface (host-logic tests on CPU), restore afterwards."""
     import minimagen_b200.ops as ops_mod

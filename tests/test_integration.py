@@ -1,6 +1,8 @@
 """Boundary proof through the REFERENCE's own callers (SURVEY.md 8b / 8f-3): INTEGRATION.md's snippet run verbatim, and a
 Training Directory round trip through the reference's `generate.load_minimagen` after `install_as_minimagen()`.
-Needs /root/reference (build container only); runs in a subprocess because it re-binds sys.modules['minimagen*']."""
+Needs a checkout of the original MinImagen project (oracle/reference.py, $MINIMAGEN_REFERENCE) -- its own generate.py and
+training.py are what is exercised, so no stored fixture can stand in for it and it skips without one; runs in a subprocess
+because it re-binds sys.modules['minimagen*']."""
 import json
 import os
 import subprocess
