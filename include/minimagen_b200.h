@@ -253,6 +253,23 @@ int mi_step_finalize(const float* x, long long n, int unnormalize, float* out, v
 int mi_q_sample(const float* x0, const float* noise, const long long* t, const float* sqrt_alphas_cumprod,
                 const float* sqrt_one_minus_alphas_cumprod, int B, int n, float post_scale, float post_shift,
                 float* out, void* stream);
+/* Inpainting (RePaint resampling), one replay = step -> mi_inpaint_blend -> mi_inpaint_advance.  x [B][C][H][W] fp32 is
+ * updated in place; known (the normalised image to keep), z_known and z_renoise have its shape; mask uint8 [B][mask_h][mask_w]
+ * (nonzero = known pixel) is sampled nearest-neighbour: m[b][i][j] = mask[b][i*mask_h/H][j*mask_w/W].  t int64 [B], u int32 [1]
+ * (the resample round at t), U resample rounds per timestep (1 at t == 0); sqrt_alphas[t] = sqrt(1 - beta_t),
+ * sqrt_betas[t] = sqrt(beta_t).  With U_t = (t > 0 ? U : 1):
+ *   prime:            x = m ? sqrt_acp[t] known + sqrt_1macp[t] z_known : x                 (before the first step)
+ *   u < U_t - 1:      x = m ? sqrt_acp[t] known + sqrt_1macp[t] z_known : sqrt_alphas[t] x + sqrt_betas[t] z_renoise
+ *   else, t > 0:      x = m ? sqrt_acp[t-1] known + sqrt_1macp[t-1] z_known : x
+ *   else (t == 0):    x = m ? known : x
+ * Products and sums are un-fused, in torch's order (a*x + b*z).  Pointers must be non-NULL, sizes positive, U >= 1. */
+int mi_inpaint_blend(float* x, const float* known, const unsigned char* mask, int mask_h, int mask_w, const float* z_known,
+                     const float* z_renoise, const long long* t, const int* u, int U, int prime,
+                     const float* sqrt_alphas_cumprod, const float* sqrt_one_minus_alphas_cumprod, const float* sqrt_alphas,
+                     const float* sqrt_betas, int B, int C, int H, int W, void* stream);
+/* After mi_inpaint_blend: if that step renoised (u < U_t - 1, decided on t[0]) u += 1, else u = 0 and t[b] = max(t[b] - 1, 0).
+ * A launch of its own: the blend's CTAs all read t and u. */
+int mi_inpaint_advance(long long* t, int* u, int U, int B, void* stream);
 
 /* ------------------------------------------------------------------------------------------------- training (backward)
  * The training side of the same path: Imagen.forward / _p_losses (Imagen.py:512-650) back-propagate through Unet.forward

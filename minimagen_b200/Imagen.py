@@ -7,11 +7,14 @@ x0 prediction, EXACT per-image dynamic-threshold quantile (radix select), poster
 (both U-Net passes + epilogue) is optionally replayed from a CUDA graph so the ~10^3 kernel launches per step cost
 nothing on the host.
 
-Two additions that the reference does not have (both optional, defaults reproduce the reference):
+Three additions that the reference does not have (all optional, defaults reproduce the reference):
   * `noise_fn(kind, shape, step)`  -- inject the Gaussian draws (x_T, per-step noise, low-res augmentation noise) so that
     a CPU oracle and this GPU path consume identical numbers (CPU mt19937 and CUDA Philox streams differ);
   * data-parallel sampling over `torch.distributed` ranks: the batch is sharded, each rank runs the whole cascade on
-    its shard, ONE NCCL all-gather assembles the finished images (`sample(..., distributed=True)`).
+    its shard, ONE NCCL all-gather assembles the finished images (`sample(..., distributed=True)`);
+  * text-guided inpainting (`sample(..., inpaint_images=, inpaint_masks=, inpaint_resample_times=)`, the keywords of
+    imagen-pytorch): the masked pixels are kept from the given images, the rest is generated, with RePaint resampling;
+    the blend and the resample counter run on the device inside the captured step (csrc/step.cu, DESIGN.md 4.6).
 """
 from contextlib import contextmanager
 from typing import Callable, List, Literal, Tuple, Union
@@ -47,19 +50,29 @@ class _StepGraph:
          noise  [B, C, s, s]  the step's Gaussian draw: drawn INSIDE the graph (graph-safe Philox) unless the caller
                               injects noise, in which case it is copied here before each replay;
          cond   static copies of text_embeds / text_mask / lowres_cond_img / lowres_noise_times (`set_cond` refreshes them).
-    A whole sampling loop is then `set x, t; replay() * T` -- no per-step host-side tensor ops."""
+    A whole sampling loop is then `set x, t; replay() * T` -- no per-step host-side tensor ops.
+    An inpainting step graph adds the RePaint blend and its counter after the step:
+         known  [B, C, s, s]  the normalised image to keep; mask uint8 [B, mh, mw] (nonzero = known), both refreshed by
+                              `set_cond`;
+         z_known, z_renoise   the blend's two Gaussian draws (in-graph, or copied in like `noise`);
+         u      [1] int32     the resample round at t, advanced with t by mi_inpaint_advance."""
 
     def __init__(self):
         self.graph = None
         self.x = self.t = self.noise = None
+        self.known = self.mask = self.z_known = self.z_renoise = self.u = None
         self.cond = {}
         self.inject_noise = False
         self.unet = None
 
-    def set_cond(self, **tensors):
+    def set_cond(self, known=None, mask=None, **tensors):
         for k, v in tensors.items():
             if v is not None:
                 self.cond[k].copy_(v)
+        if known is not None:
+            self.known.copy_(known)
+        if mask is not None:
+            self.mask.copy_(mask)
         self.refresh_static()
 
     def refresh_static(self):
@@ -281,13 +294,14 @@ class Imagen(nn.Module):
 
     # -------------------------------------------------------------------------------------------- sampling loop
     def _graph_key(self, unet, shape, noise_scheduler, text_embeds, text_mask, lowres_cond_img, lowres_noise_times,
-                   cond_scale):
+                   cond_scale, inpaint=None):
         sig = lambda v: None if v is None else (tuple(v.shape), str(v.dtype))
         p0 = next(unet.parameters())
+        inpaint_sig = None if inpaint is None else (tuple(inpaint[1].shape), int(inpaint[2]))   # (mask shape, U)
         return (id(unet), tuple(shape), float(cond_scale), bool(self.cfg_batched), exists(self.noise_fn),
                 noise_scheduler.num_timesteps, sig(text_embeds), sig(text_mask), sig(lowres_cond_img),
                 sig(lowres_noise_times), p0.data_ptr(), sum(p._version for p in unet.parameters()),
-                self.dynamic_thresholding_percentile)
+                self.dynamic_thresholding_percentile, inpaint_sig)
 
     def clear_graphs(self):
         """Drop the captured step graphs (and the activation memory their pools hold)."""
@@ -297,17 +311,19 @@ class Imagen(nn.Module):
         self.max_cached_graphs = 4
 
     def _step_graph(self, unet, shape, *, noise_scheduler, text_embeds, text_mask, lowres_cond_img,
-                    lowres_noise_times, cond_scale):
+                    lowres_noise_times, cond_scale, inpaint=None):
         """The captured step for this (unet, shape, conditioning signature, weights version): captured once, then reused by
-        every later sampling loop of the same signature; the conditioning tensors are refreshed in its static buffers."""
+        every later sampling loop of the same signature; the conditioning tensors are refreshed in its static buffers.
+        `inpaint` = (known, mask uint8, U) captures the inpainting step instead: step, RePaint blend, advance of (t, u)."""
         device = self.device
         key = self._graph_key(unet, shape, noise_scheduler, text_embeds, text_mask, lowres_cond_img,
-                              lowres_noise_times, cond_scale)
+                              lowres_noise_times, cond_scale, inpaint)
         cond = dict(text_embeds=text_embeds, text_mask=text_mask, lowres_cond_img=lowres_cond_img,
                     lowres_noise_times=lowres_noise_times)
+        known, mask, U = inpaint if inpaint is not None else (None, None, None)
         g = self._graphs.get(key)
         if g is not None:
-            g.set_cond(**cond)
+            g.set_cond(known=known, mask=mask, **cond)
             return g
         if len(self._graphs) >= self.max_cached_graphs:
             self._graphs.pop(next(iter(self._graphs))).release()
@@ -322,12 +338,26 @@ class Imagen(nn.Module):
                   **{k: g.cond.get(k) for k in cond})
         g.refresh_static()
         ops = get_ops()
+        if inpaint is not None:
+            g.known, g.mask = known.clone(), mask.clone()
+            g.z_known = torch.zeros(shape, dtype=F32, device=device)
+            g.z_renoise = torch.zeros(shape, dtype=F32, device=device)
+            g.u = torch.zeros((1,), dtype=torch.int32, device=device)
+            sa, sb = noise_scheduler.inpaint_tables(device)
 
         def body():
             if not g.inject_noise:
                 g.noise.normal_()                       # the reference's randn_like(x) (Imagen.py:361), graph-safe Philox
+                if inpaint is not None:
+                    g.z_renoise.normal_()
+                    g.z_known.normal_()
             self._step(unet, g.x, g.t, g.noise, out=g.x, **kw)
-            ops.step_advance_t(g.t, shape[0])           # t <- max(t - 1, 0): the next loop iteration's timestep
+            if inpaint is None:
+                ops.step_advance_t(g.t, shape[0])       # t <- max(t - 1, 0): the next loop iteration's timestep
+            else:
+                ops.inpaint_blend(g.x, g.known, g.mask, g.z_known, g.z_renoise, g.t, g.u, U, 0,
+                                  noise_scheduler.sqrt_alphas_cumprod, noise_scheduler.sqrt_one_minus_alphas_cumprod, sa, sb)
+                ops.inpaint_advance(g.t, g.u, U, shape[0])   # (t, u) of the next replay
 
         # warm-up on a side stream (packs weights, sizes the caching allocator), then capture
         side = torch.cuda.Stream(device=device)
@@ -342,12 +372,68 @@ class Imagen(nn.Module):
         self._graphs[key] = g
         return g
 
+    @staticmethod
+    def _inpaint_schedule(T, U):
+        """(t, u) of every step of an inpainting loop: U resample rounds at each t > 0, one at t = 0."""
+        return [(t, u) for t in reversed(range(T)) for u in range(U if t > 0 else 1)]
+
+    def _inpaint_loop(self, unet, shape, img, inpaint, max_steps, kw):
+        """The sampling loop with RePaint inpainting (DESIGN.md 4.6): prime the known region at T-1, then per step of the
+        schedule x <- step(x, t), blend (renoise back to t and redo, or paste the known region at t-1 / at 0), advance
+        (t, u).  Injected noise is drawn as ('step', key), ('renoise', key) if the step renoises, ('inpaint', key) unless
+        it is the final paste, with key = t * U + u; the prime draws ('inpaint', -1)."""
+        known, mask, U = inpaint
+        ops = get_ops()
+        sch = kw['noise_scheduler']
+        T, B, device = sch.num_timesteps, shape[0], img.device
+        sa, sb = sch.inpaint_tables(device)
+        tabs = (sch.sqrt_alphas_cumprod, sch.sqrt_one_minus_alphas_cumprod, sa, sb)
+        steps = self._inpaint_schedule(T, U)
+        if exists(max_steps):
+            steps = steps[:max_steps]
+        renoises = lambda t, u: u < (U if t > 0 else 1) - 1
+        z_prime = self._noise('inpaint', shape, -1, device)
+        if self.use_cuda_graph and img.is_cuda and len(steps) > 2:
+            g = self._step_graph(unet, tuple(shape), inpaint=inpaint, **kw)
+            g.x.copy_(img)
+            g.t.fill_(T - 1)
+            g.u.zero_()
+            g.z_known.copy_(z_prime)
+            ops.inpaint_blend(g.x, g.known, g.mask, g.z_known, g.z_renoise, g.t, g.u, U, 1, *tabs)
+            for t, u in steps:
+                if g.inject_noise:
+                    key = t * U + u
+                    g.noise.copy_(self._noise('step', shape, key, device))
+                    if renoises(t, u):
+                        g.z_renoise.copy_(self._noise('renoise', shape, key, device))
+                    if t > 0:
+                        g.z_known.copy_(self._noise('inpaint', shape, key, device))
+                g.replay()                              # x <- blend(step(x)) in place, (t, u) advanced
+            return g.x
+        t_dev = torch.full((B,), T - 1, dtype=torch.long, device=device)
+        u_dev = torch.zeros((1,), dtype=torch.int32, device=device)
+        z_known = z_renoise = z_prime                   # z_renoise is only read by a renoising blend
+        x = img.contiguous().clone()                    # the prime blends in place; img may be the caller's noise_fn draw
+        ops.inpaint_blend(x, known, mask, z_known, z_renoise, t_dev, u_dev, U, 1, *tabs)
+        for t, u in steps:
+            key = t * U + u
+            x = self._step(unet, x, t_dev, self._noise('step', shape, key, device), **kw)
+            if renoises(t, u):
+                z_renoise = self._noise('renoise', shape, key, device)
+            if t > 0:
+                z_known = self._noise('inpaint', shape, key, device)
+            ops.inpaint_blend(x, known, mask, z_known, z_renoise, t_dev, u_dev, U, 0, *tabs)
+            ops.inpaint_advance(t_dev, u_dev, U, B)
+        return x
+
     @torch.no_grad()
     def _p_sample_loop(self, unet, shape, *, noise_scheduler, text_embeds=None, text_mask=None, lowres_cond_img=None,
-                       lowres_noise_times=None, cond_scale=1., max_steps=None, out=None):
+                       lowres_noise_times=None, cond_scale=1., max_steps=None, out=None, inpaint=None):
         """Reverse diffusion from x_T ~ N(0, I) to x_0 (reference Imagen.py:372-420).  `max_steps` (not in the
         reference) stops after that many iterations -- used by the benchmark / parity harness; `out` (not in the
-        reference) receives the finished images (e.g. this rank's slot of the all-gather buffer)."""
+        reference) receives the finished images (e.g. this rank's slot of the all-gather buffer).  `inpaint` (not in the
+        reference) = (known [B, C, s, s] normalised fp32, mask uint8 [B, mh, mw], U) runs the inpainting loop
+        (`_inpaint_loop`); `max_steps` then counts its (T - 1) * U + 1 steps."""
         device = self.device
         with N.device_of(self._temp):
             ops = get_ops()
@@ -362,7 +448,9 @@ class Imagen(nn.Module):
 
             kw = dict(noise_scheduler=noise_scheduler, text_embeds=text_embeds, text_mask=text_mask,
                       lowres_cond_img=lowres_cond_img, lowres_noise_times=lowres_noise_times, cond_scale=cond_scale)
-            if self.use_cuda_graph and img.is_cuda and len(timesteps) > 2:
+            if exists(inpaint):
+                img = self._inpaint_loop(unet, shape, img, inpaint, max_steps, kw)
+            elif self.use_cuda_graph and img.is_cuda and len(timesteps) > 2:
                 g = self._step_graph(unet, tuple(shape), **kw)
                 g.x.copy_(img)
                 g.t.copy_(timesteps[0])
@@ -385,21 +473,44 @@ class Imagen(nn.Module):
     @eval_decorator
     def sample(self, texts: List[str] = None, text_masks=None, text_embeds=None, cond_scale: float = 1.,
                lowres_sample_noise_level: float = None, return_pil_images: bool = False, device=None,
-               distributed: bool = False):
+               distributed: bool = False, inpaint_images=None, inpaint_masks=None, inpaint_resample_times: int = 5):
         """Generate images (reference Imagen.py:422-510).  With `distributed=True` inside an initialised
         torch.distributed (NCCL) job, rank r samples rows [r*b/G, (r+1)*b/G) of the conditioning; the last stage's
         finalize kernel writes its images straight into this rank's slot of the gather buffer and ONE in-place
-        all-gather returns the full batch on every rank."""
+        all-gather returns the full batch on every rank.
+        Inpainting (not in the reference; the keywords of imagen-pytorch): `inpaint_images` float (b, channels, H, H) in
+        [0, 1] and `inpaint_masks` bool (b, H, H), True = keep that pixel of the image, False = generate it.  Every stage
+        keeps the known region of the image resized to its size and re-runs each timestep `inpaint_resample_times` times
+        (RePaint resampling), so each stage takes (T - 1) * inpaint_resample_times + 1 steps."""
         device = torch.device(default(device, self.device))
         self._reset_unets_all_one_device(device=device)
         if self._temp.device != device:
             self.to(device)
         with N.device_of(self._temp):
             return self._sample_impl(texts, text_masks, text_embeds, cond_scale, lowres_sample_noise_level,
-                                     return_pil_images, device, distributed)
+                                     return_pil_images, device, distributed, inpaint_images, inpaint_masks,
+                                     inpaint_resample_times)
+
+    def _check_inpaint_args(self, inpaint_images, inpaint_masks, inpaint_resample_times, batch):
+        U = inpaint_resample_times
+        assert isinstance(U, int) and not isinstance(U, bool) and U >= 1, \
+            f'inpaint_resample_times must be an int >= 1, got {U!r}'
+        assert exists(inpaint_images) == exists(inpaint_masks), \
+            'inpaint_images and inpaint_masks must be given together'
+        if not exists(inpaint_images):
+            return
+        assert torch.is_tensor(inpaint_images) and inpaint_images.is_floating_point() and inpaint_images.dim() == 4, \
+            f'inpaint_images must be a float tensor (b, {self.channels}, h, h)'
+        b, c, h, w = inpaint_images.shape
+        assert b == batch and c == self.channels and h == w, \
+            f'inpaint_images must be ({batch}, {self.channels}, h, h), got {tuple(inpaint_images.shape)}'
+        assert torch.is_tensor(inpaint_masks) and inpaint_masks.dtype == torch.bool and inpaint_masks.dim() == 3 \
+            and inpaint_masks.shape[0] == batch, f'inpaint_masks must be a bool tensor ({batch}, h, h)'
+        assert tuple(inpaint_masks.shape[-2:]) == (h, w), \
+            f'inpaint_masks size {tuple(inpaint_masks.shape[-2:])} differs from the inpaint_images size {(h, w)}'
 
     def _sample_impl(self, texts, text_masks, text_embeds, cond_scale, lowres_sample_noise_level, return_pil_images,
-                     device, distributed):
+                     device, distributed, inpaint_images=None, inpaint_masks=None, inpaint_resample_times=5):
         if exists(texts) and not exists(text_embeds):
             text_embeds, text_masks = t5_encode_text(texts, name=self.text_encoder_name)
             text_embeds, text_masks = map(lambda t: t.to(device), (text_embeds, text_masks))
@@ -407,6 +518,8 @@ class Imagen(nn.Module):
         assert exists(text_embeds), 'text or text encodings must be passed into Imagen'
         assert not (exists(text_embeds) and text_embeds.shape[-1] != self.text_embed_dim), \
             f'invalid text embedding dimension being passed in (should be {self.text_embed_dim})'
+        self._check_inpaint_args(inpaint_images, inpaint_masks, inpaint_resample_times, text_embeds.shape[0])
+        inpainting = exists(inpaint_images)
 
         world, rank = 1, 0
         if distributed:
@@ -418,12 +531,18 @@ class Imagen(nn.Module):
             per = full_b // world
             text_embeds = text_embeds[rank * per:(rank + 1) * per]
             text_masks = text_masks[rank * per:(rank + 1) * per] if exists(text_masks) else None
+            if inpainting:
+                inpaint_images = inpaint_images[rank * per:(rank + 1) * per]
+                inpaint_masks = inpaint_masks[rank * per:(rank + 1) * per]
 
         batch_size = text_embeds.shape[0]
         text_embeds = text_embeds.to(device=device, dtype=F32).contiguous()
         text_masks = text_masks.to(device).contiguous() if exists(text_masks) else None
         lowres_sample_noise_level = default(lowres_sample_noise_level, self.lowres_sample_noise_level)
         ops = get_ops()
+        if inpainting:
+            inpaint_images = inpaint_images.to(device=device, dtype=F32).contiguous()
+            inpaint_masks = inpaint_masks.to(device=device, dtype=torch.uint8).contiguous()
 
         img = None
         gathered = None
@@ -445,6 +564,12 @@ class Imagen(nn.Module):
                                  noised)
                     lowres_cond_img = noised
                 shape = (batch_size, self.channels, image_size, image_size)
+                inpaint = None
+                if inpainting:
+                    # the image to keep at this stage's size, normalised like the sampling state (once per stage)
+                    known = resize_image_to(inpaint_images, image_size, pad_mode='reflect')
+                    known = self.normalize_img(known).to(F32).contiguous()
+                    inpaint = (known, inpaint_masks, inpaint_resample_times)
                 slot = None
                 if distributed and world > 1 and unet_number == n_stages:
                     # the last stage finalises straight into this rank's slot of the all-gather buffer (no staging copy)
@@ -453,7 +578,7 @@ class Imagen(nn.Module):
                 img = self._p_sample_loop(unet, shape, text_embeds=text_embeds, text_mask=text_masks,
                                           cond_scale=cond_scale, lowres_cond_img=lowres_cond_img,
                                           lowres_noise_times=lowres_noise_times, noise_scheduler=noise_scheduler,
-                                          out=slot)
+                                          out=slot, inpaint=inpaint)
 
         outputs = img
         if gathered is not None:

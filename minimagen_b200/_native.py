@@ -55,6 +55,8 @@ SIGNATURES = {
     "mi_step_advance_t": [_P, _I, _P],
     "mi_step_finalize": [_P, _L, _I, _P, _P],
     "mi_q_sample": [_P, _P, _P, _P, _P, _I, _I, _F, _F, _P, _P],
+    "mi_inpaint_blend": [_P, _P, _P, _I, _I, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _I, _I, _I, _I, _P],
+    "mi_inpaint_advance": [_P, _P, _I, _I, _P],
     # training side (backward)
     "mi_gemm_f32": [_P, _P, _P, _I, _I, _I, _L, _L, _L, _L, _L, _L, _I, _I, _L, _L, _L, _L, _L, _L, _F, _I, _P],
     "mi_colsum_f32": [_P, _L, _I, _P, _I, _P],

@@ -307,6 +307,17 @@ int mi_q_sample(const float* x0, const float* noise, const long long* t, const f
                 int n, float post_scale, float post_shift, float* out, void* stream) {
     return check(mi::q_sample(x0, noise, t, tab_a, tab_b, B, n, post_scale, post_shift, out, S(stream)), "mi_q_sample");
 }
+int mi_inpaint_blend(float* x, const float* known, const unsigned char* mask, int mask_h, int mask_w, const float* z_known,
+                     const float* z_renoise, const long long* t, const int* u, int U, int prime,
+                     const float* sqrt_alphas_cumprod, const float* sqrt_one_minus_alphas_cumprod, const float* sqrt_alphas,
+                     const float* sqrt_betas, int B, int C, int H, int W, void* stream) {
+    return check(mi::inpaint_blend(x, known, mask, mask_h, mask_w, z_known, z_renoise, t, u, U, prime, sqrt_alphas_cumprod,
+                                   sqrt_one_minus_alphas_cumprod, sqrt_alphas, sqrt_betas, B, C, H, W, S(stream)),
+                 "mi_inpaint_blend");
+}
+int mi_inpaint_advance(long long* t, int* u, int U, int B, void* stream) {
+    return check(mi::inpaint_advance(t, u, U, B, S(stream)), "mi_inpaint_advance");
+}
 
 int mi_gemm_f32(const float* A, const float* B, float* C, int M, int N, int K, long long a_sm, long long a_sk,
                 long long b_sk, long long b_sn, long long c_sm, long long c_sn, int Z1, int Z2, long long a_b1,

@@ -77,6 +77,11 @@ int step_advance_t(long long* t, int B, cudaStream_t st);
 int step_finalize(const float* x, long long n, int unnormalize, float* out, cudaStream_t st);
 int q_sample(const float* x0, const float* noise, const long long* t, const float* tab_a, const float* tab_b, int B,
              int n_per_img, float post_scale, float post_shift, float* out, cudaStream_t st);
+int inpaint_blend(float* x, const float* known, const unsigned char* mask, int mask_h, int mask_w, const float* z_known,
+                  const float* z_renoise, const long long* t, const int* u, int U, int prime, const float* tab_acp,
+                  const float* tab_1macp, const float* tab_sa, const float* tab_sb, int B, int C, int H, int W,
+                  cudaStream_t st);
+int inpaint_advance(long long* t, int* u, int U, int B, cudaStream_t st);
 
 // backward.cu: fp32 backward kernels of the training side (SURVEY 8f-2)
 int gemm_f32(const float* A, const float* B, float* C, int M, int N, int K, long long a_sm, long long a_sk, long long b_sk,

@@ -451,7 +451,87 @@ __global__ void q_sample_kernel(const float* __restrict__ x0, const float* __res
     out[idx] = v;
 }
 
+// ------------------------------------------------------------------------------------------------ inpainting (RePaint)
+// One replay of an inpainting sampling loop is  step (x <- x_{t-1}) -> inpaint_blend -> inpaint_advance.  With U resample
+// rounds per timestep (1 at t == 0) and the round counter u on the device, the blend after the step of (t, u) is
+//   u < U_t - 1:  x <- m ? sqrt_acp[t] K + sqrt_1macp[t] z_k     : sqrt(1 - beta_t) x + sqrt(beta_t) z_r   (back to t, redo)
+//   else t > 0:   x <- m ? sqrt_acp[t-1] K + sqrt_1macp[t-1] z_k : x                                      (known part at t-1)
+//   else:         x <- m ? K : x                                                                          (final paste)
+// and prime = 1 gives the blend before the first step:  x <- m ? sqrt_acp[t] K + sqrt_1macp[t] z_k : x.
+// m[b, i, j] = mask[b, (i * mask_h) / H, (j * mask_w) / W]: nearest-neighbour sampling of the caller's mask at its own
+// resolution.  Products and sums un-fused, in the order torch evaluates a * x + b * z.  x is updated in place; every element
+// is read and written by the same thread.  One thread per pixel, looping over the channels: the mask index (three 32-bit
+// divisions; the launcher keeps H * mask_h and W * mask_w below 2^32) is computed once per pixel, not once per element.
+__global__ void __launch_bounds__(256)
+inpaint_blend_kernel(float* x, const float* __restrict__ known, const unsigned char* __restrict__ mask, int mask_h,
+                     int mask_w, const float* __restrict__ z_known, const float* __restrict__ z_renoise,
+                     const long long* __restrict__ t, const int* __restrict__ u, int U, int prime,
+                     const float* __restrict__ tab_acp, const float* __restrict__ tab_1macp,
+                     const float* __restrict__ tab_sa, const float* __restrict__ tab_sb, int C, int H, int W) {
+    pdl_wait();
+    pdl_trigger();
+    const int b = blockIdx.y;
+    const unsigned hw = (unsigned)H * W;
+    const unsigned p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= hw) return;
+    const unsigned row = p / (unsigned)W, col = p - row * (unsigned)W;
+    const unsigned mr = row * (unsigned)mask_h / (unsigned)H, mc = col * (unsigned)mask_w / (unsigned)W;
+    const bool m = mask[((long long)b * mask_h + mr) * mask_w + mc] != 0;
+    const long long tb = t[b];
+    const int ut = tb > 0 ? U : 1;
+    // 0: x = a K + c z_k at ta (prime / renoise / t > 0, masked);  1: x = K (final paste, masked);
+    // 2: x = sa x + sb z_r (renoise, unmasked);  3: x unchanged
+    const bool renoise = !prime && *u < ut - 1;
+    const long long ta = (prime || renoise) ? tb : tb - 1;
+    const int op = m ? ((prime || renoise || tb > 0) ? 0 : 1) : (renoise ? 2 : 3);
+    if (op == 3) return;
+    const float a = op == 0 ? tab_acp[ta] : (op == 2 ? tab_sa[tb] : 0.f);
+    const float c = op == 0 ? tab_1macp[ta] : (op == 2 ? tab_sb[tb] : 0.f);
+    const float* src = op == 2 ? x : known;
+    const float* z = op == 2 ? z_renoise : z_known;
+    const long long base = (long long)b * C * hw + p;
+    for (int ch = 0; ch < C; ++ch) {
+        const long long idx = base + (long long)ch * hw;
+        x[idx] = op == 1 ? known[idx] : __fadd_rn(__fmul_rn(a, src[idx]), __fmul_rn(c, z[idx]));
+    }
+}
+
+// After the blend: a renoising round stays at t (u += 1), otherwise u = 0 and t = max(t - 1, 0).  Every CTA of the blend
+// reads t and u, so they are advanced by this separate single-CTA launch.  The rounds are counted for the whole batch (one
+// sampling loop: every image is at the same t); the decision reads t[0].
+__global__ void __launch_bounds__(128) inpaint_advance_kernel(long long* t, int* u, int U, int B) {
+    pdl_wait();
+    pdl_trigger();
+    const int uu = *u;
+    const bool renoised = uu < (t[0] > 0 ? U : 1) - 1;
+    __syncthreads();                                   // every thread has read t[0] and u before anyone writes them
+    if (!renoised)
+        for (int i = threadIdx.x; i < B; i += blockDim.x) t[i] = t[i] > 0 ? t[i] - 1 : 0;
+    if (threadIdx.x == 0) *u = renoised ? uu + 1 : 0;
+}
+
 }  // namespace
+
+int inpaint_blend(float* x, const float* known, const unsigned char* mask, int mask_h, int mask_w, const float* z_known,
+                  const float* z_renoise, const long long* t, const int* u, int U, int prime, const float* tab_acp,
+                  const float* tab_1macp, const float* tab_sa, const float* tab_sb, int B, int C, int H, int W,
+                  cudaStream_t st) {
+    if (!x || !known || !mask || !z_known || !z_renoise || !t || !u || !tab_acp || !tab_1macp || !tab_sa || !tab_sb)
+        return -1;
+    if (mask_h <= 0 || mask_w <= 0 || U < 1 || B <= 0 || C <= 0 || H <= 0 || W <= 0) return -1;
+    const long long u32 = 1LL << 32;
+    if ((long long)H * W >= u32 || (long long)H * mask_h >= u32 || (long long)W * mask_w >= u32 || B > 65535) return -1;
+    dim3 grid((unsigned)(((long long)H * W + 255) / 256), B);
+    launch_k(inpaint_blend_kernel, grid, 256, 0, st, x, known, mask, mask_h, mask_w, z_known, z_renoise, t, u, U, prime,
+             tab_acp, tab_1macp, tab_sa, tab_sb, C, H, W);
+    return cudaGetLastError() == cudaSuccess ? 0 : -2;
+}
+
+int inpaint_advance(long long* t, int* u, int U, int B, cudaStream_t st) {
+    if (!t || !u || U < 1 || B <= 0) return -1;
+    launch_k(inpaint_advance_kernel, 1, 128, 0, st, t, u, U, B);
+    return cudaGetLastError() == cudaSuccess ? 0 : -2;
+}
 
 int step_x0(const float* x_t, const float* eps_cond, const float* eps_null, float cond_scale, const long long* t,
             const float* tab_recip, const float* tab_recipm1, int B, int n_per_img, float* x0, cudaStream_t st) {

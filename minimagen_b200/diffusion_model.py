@@ -46,6 +46,20 @@ class GaussianDiffusion(nn.Module):
         reg('posterior_mean_coef2', (1. - acp_prev) * torch.sqrt(alphas) / (1. - acp))
         # what `(0.5 * model_log_variance).exp()` (Imagen.py:370) evaluates to on the fp32 table, op by op in fp32
         reg('sigma', (0.5 * self.posterior_log_variance_clipped).exp())
+        self._inpaint_tables = {}
+
+    def inpaint_tables(self, device):
+        """(sqrt(1 - beta), sqrt(beta)) as fp32 tables on `device`: the coefficients of RePaint's step back from t-1 to t
+        (inpainting).  Computed in fp64 from the schedule like the buffers above, cached per device; deliberately not
+        buffers, so `.buffers()` / `state_dict()` are those of the reference."""
+        key = str(device)
+        tabs = self._inpaint_tables.get(key)
+        if tabs is None:
+            scale = 1000 / self.num_timesteps
+            betas = torch.linspace(scale * 0.0001, scale * 0.02, self.num_timesteps, dtype=torch.float64)
+            tabs = tuple(v.to(device=device, dtype=torch.float32) for v in (torch.sqrt(1. - betas), torch.sqrt(betas)))
+            self._inpaint_tables[key] = tabs
+        return tabs
 
     # ---- integer timestep generators (diffusion_model.py:68-87)
     def _get_times(self, batch_size, noise_level, *, device):

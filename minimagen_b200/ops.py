@@ -251,6 +251,24 @@ class NativeOps:
         N.call("mi_q_sample", N.ptr(x0), N.ptr(noise), N.ptr(t), N.ptr(tab_a), N.ptr(tab_b), B, n, float(post_scale),
                float(post_shift), N.ptr(out), N.stream())
 
+    def inpaint_blend(self, x, known, mask, z_known, z_renoise, t, u, U, prime, sqrt_acp, sqrt_1macp, sqrt_alphas,
+                      sqrt_betas):
+        """RePaint blend of one inpainting replay, in place on x [B, C, H, W]; mask uint8 [B, mh, mw] (nonzero = known pixel),
+        sampled nearest-neighbour at x's size; u int32 [1] the resample round (mi_inpaint_blend)."""
+        for nm, tt in (("x", x), ("known", known), ("z_known", z_known), ("z_renoise", z_renoise), ("sqrt_acp", sqrt_acp),
+                       ("sqrt_1macp", sqrt_1macp), ("sqrt_alphas", sqrt_alphas), ("sqrt_betas", sqrt_betas)):
+            _chk(tt, F32, nm)
+        _chk(mask, U8, "mask"); _chk(t, I64, "t"); _chk(u, torch.int32, "u")
+        B, C, H, W = x.shape
+        N.call("mi_inpaint_blend", N.ptr(x), N.ptr(known), N.ptr(mask), mask.shape[-2], mask.shape[-1], N.ptr(z_known),
+               N.ptr(z_renoise), N.ptr(t), N.ptr(u), int(U), int(prime), N.ptr(sqrt_acp), N.ptr(sqrt_1macp),
+               N.ptr(sqrt_alphas), N.ptr(sqrt_betas), B, C, H, W, N.stream())
+
+    def inpaint_advance(self, t, u, U, B):
+        """u += 1 after a renoising round, else u = 0 and t <- max(t - 1, 0) (mi_inpaint_advance)."""
+        _chk(t, I64, "t"); _chk(u, torch.int32, "u")
+        N.call("mi_inpaint_advance", N.ptr(t), N.ptr(u), int(U), B, N.stream())
+
 
     # ---------------------------------------------------------------- training side (backward kernels, fp32)
     def gemm_f32(self, A, B, C, M, N, K, a_str, b_str, c_str, Z1=1, Z2=1, a_b=(0, 0), b_b=(0, 0), c_b=(0, 0), alpha=1.0,
